@@ -2,7 +2,7 @@
 """bench.py — reads mapped / second of the B200 hot path (BASELINE.json metric), per the driver contract.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg4|cfg3|cfg2|cfg1]
-                    [--batch READS_PER_STEP] [--scaling weak|strong]
+                    [--batch READS_PER_STEP] [--scaling weak|strong] [--dump-outputs DIR]
 
 Default workload: BASELINE cfg4, the metric's own configuration (3.1 Gbp hg19-scale synthetic reference, 25-100 bp
 single-stranded damaged reads, -p 0.03); `--workload cfg3` etc. give the other BASELINE shapes.
@@ -18,6 +18,8 @@ K + W steps fit its time limit — stated in config.workload).  Every step uses 
   parity the records of one timed end-to-end chunk are compared with the CPU oracle's on the same reads (bit-exact on
          position, strand, CIGAR, MD, NM, MAPQ, X0/X1/XS, best-hit interval, scores and the work counters);
          any mismatch makes the run exit non-zero
+  --dump-outputs DIR  writes the records of the last timed chunk (rank 0) as DIR/<name>.npy, so that two builds can be
+         compared output for output on identical inputs (see dump_outputs)
 Multi-GPU: one process per GPU (torchrun), index built once on rank 0 and broadcast with NCCL, reads sharded per rank
 (weak scaling: K chunks per rank; --scaling strong: the same K chunks split over the ranks), no data-path collective.
 `--impl reference` times the CPU restatement of mapAD 0.45.0 (oracle/, all host threads): the reference itself is Rust and
@@ -156,6 +158,48 @@ def run_cpu(oix, spec, packed, n_sample, threads):
     return n / dt, dt, n, res
 
 
+DUMP_MAX_READS = 100_000
+DUMP_MAX_BYTES = 64 << 20
+
+
+def _gather(pool, offs, lens):
+    """pool[offs[0]:offs[0]+lens[0]], pool[offs[1]:...], ... concatenated"""
+    offs, lens = offs.astype(np.int64).ravel(), lens.astype(np.int64).ravel()
+    starts = np.cumsum(lens) - lens
+    return pool[np.repeat(offs - starts, lens) + np.arange(int(lens.sum()))]
+
+
+def dump_outputs(res, out_dir):
+    """Writes what a caller of the timed path receives for one chunk as out_dir/<name>.npy: every per-read record field
+    (integers as float64, f32 scores as float32; alternative hits as alt_<field>, shape (n, 2)) and, per read in read
+    order, the CIGAR words and MD text of its primary alignment followed by those of its alternative hits (float32;
+    the *_len fields split them).  Pool offsets are left out: they only say where the library put the strings.  Of
+    flags only bit 0 (search limit hit) is kept: bit 1 (went through the retry lane) depends on what else was in flight.
+    Chunks of more than DUMP_MAX_READS reads are sampled with a fixed seed; read_index holds the sampled reads."""
+    rec = res.records
+    n = len(rec)
+    idx = np.arange(n) if n <= DUMP_MAX_READS else np.sort(np.random.default_rng(0).choice(n, DUMP_MAX_READS, replace=False))
+    rec = rec[idx]
+    alts = rec["alts"]
+    out = {"read_index": idx.astype(np.float64)}
+    for table, prefix in ((rec, ""), (alts, "alt_")):
+        for f in table.dtype.names:
+            if f in ("alts", "cigar_off", "md_off", "hit_off"):
+                continue
+            v = table[f] & 1 if f == "flags" else table[f]
+            out[prefix + f] = v.astype(np.float32 if v.dtype == np.float32 else np.float64)
+    for name, pool, off, ln in (("cigar", res.cigar, "cigar_off", "cigar_len"), ("md", np.frombuffer(res.text, np.uint8), "md_off", "md_len")):
+        offs = np.concatenate([rec[off][:, None], alts[off]], axis=1)
+        lens = np.concatenate([rec[ln][:, None], alts[ln]], axis=1)
+        out[name] = _gather(pool, offs, lens).astype(np.float32)
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit("bench.py: --dump-outputs would write %d bytes (limit %d)" % (total, DUMP_MAX_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ---------------------------------------------------------------------------------------------------------------------
 # reference arm (CPU restatement; this process never loads the product library)
 # ---------------------------------------------------------------------------------------------------------------------
@@ -219,7 +263,10 @@ def main():
     ap.add_argument("--cpu-sample", type=int, default=0)
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the records of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -316,11 +363,11 @@ def main():
         mp.set_stream(st.cuda_stream)
     keep_result = {}
 
-    def run_pipelined(chunk_ids, resident, keep=None):
+    def run_pipelined(chunk_ids, resident, keep=()):
         """Maps the given chunks, round-robin over the handles, one host thread per handle.
         resident=True (one chunk per handle): phase U stages every chunk in HBM through the C ABI (timed on the host clock),
         phase R runs them from HBM (timed with CUDA events and on the host clock); otherwise a single phase maps from host buffers.
-        keep: chunk id whose full result (records + CIGAR/MD pools) is copied for the parity check.
+        keep: chunk ids whose full result (records + CIGAR/MD pools) is copied for the parity check and --dump-outputs.
         Returns (device seconds of phase R from first start to last end event, per-chunk stats, wall seconds of R, wall seconds of U)."""
         per = [[] for _ in mappers]
         for k, cid in enumerate(chunk_ids):
@@ -366,7 +413,7 @@ def main():
                     recs = abi._as_array(res.records, res.n_reads, abi.RECORD_DTYPE)
                     results[cid] = dict(recs=recs, ms_search=res.ms_search, ms_prologue=res.ms_prologue, ms_epilogue=res.ms_epilogue,
                                         ms_total=res.ms_total, launches=int(res.gpu_launches), n_cigar=int(res.n_cigar), n_text=int(res.n_text))
-                    if keep is not None and cid == keep:
+                    if cid in keep:
                         keep_result[cid] = abi.BatchResult(res)
                 ev1[h].record(streams[h])
             except Exception as e:  # noqa: BLE001
@@ -397,7 +444,8 @@ def main():
     sampler.start()
     # ---- timed pass: phase U (host buffers -> HBM through the C ABI), phase R (run from HBM) ----
     resident_ok = len(timed_ids) <= len(mappers)
-    dev_s, results, wall_r, wall_u = run_pipelined(timed_ids, resident=resident_ok, keep=timed_ids[0] if rank == 0 else None)
+    keep = ({timed_ids[0], timed_ids[-1]} if args.dump_outputs else {timed_ids[0]}) if rank == 0 else ()
+    dev_s, results, wall_r, wall_u = run_pipelined(timed_ids, resident=resident_ok, keep=keep)
     dev_ms = dev_s * 1e3
     wall_resident = wall_r
     e2e_wall = wall_u + wall_r
@@ -507,6 +555,8 @@ def main():
                                  "first": bad[0][1] if bad else None}
                 if bad:
                     rc = 3
+        if args.dump_outputs:
+            dump_outputs(keep_result[timed_ids[-1]], args.dump_outputs)
         print(json.dumps(out))
     for mp in mappers:
         mp.close()
