@@ -245,6 +245,15 @@ MAPAD_DEV uint8_t rank_base(int r) { return (uint8_t)("$ACGTX"[r]); }  // get_re
 MAPAD_DEV uint8_t complement_base(uint8_t b) {
   switch (b) { case 'A': return 'T'; case 'T': return 'A'; case 'C': return 'G'; case 'G': return 'C'; default: return b; }
 }
+// bio::alphabets::dna::complement: also pairs the IUPAC codes (R-Y, K-M, B-V, D-H; S, W, N map to themselves).  MD reports
+// the reference's original symbol (record.rs:301-321), complemented like a base on the reverse strand.
+MAPAD_DEV uint8_t complement_iupac(uint8_t b) {
+  switch (b) {
+    case 'R': return 'Y'; case 'Y': return 'R'; case 'K': return 'M'; case 'M': return 'K';
+    case 'B': return 'V'; case 'V': return 'B'; case 'D': return 'H'; case 'H': return 'D';
+    default: return complement_base(b);
+  }
+}
 
 // SampledSuffixArray::get.  `steps` counts LF steps + the final sample / extra-row read (W of SURVEY §8d).
 template <bool WIDE>

@@ -205,10 +205,10 @@ MAPAD_DEV void bam_fields_pass(const DevIndex& ix, const mapad_edit_op* ops, uin
     if (op.kind == MAPAD_ED_MATCH) num_matches += 1;
     else if (op.kind == MAPAD_ED_MISMATCH) {
       emit_num(num_matches);
-      emit_char((char)(backward ? complement_base(op.base) : op.base));
+      emit_char((char)(backward ? complement_iupac(op.base) : op.base));
       num_matches = 0;
     } else if (op.kind == MAPAD_ED_DELETION) {
-      char b = (char)(backward ? complement_base(op.base) : op.base);
+      char b = (char)(backward ? complement_iupac(op.base) : op.base);
       if (have_last && last_is_del) emit_char(b);
       else { emit_num(num_matches); emit_char('^'); emit_char(b); }
       num_matches = 0;

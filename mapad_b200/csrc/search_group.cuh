@@ -289,6 +289,29 @@ struct GroupWorkspace {
     }
     return Grp<G>::shfl(got, 0);
   }
+  // Group start: both base chunks or none, and no pressure while waiting.  Launches of several handles share the pool and
+  // each may start up to n_chunks / 4 groups, so two launches can hold every chunk as base chunks; the others' groups then
+  // wait until those launches exit.  Groups that each held one chunk while waiting for a second could together hold the
+  // rest of the pool, and pressure published by a group that runs no read would hold back the groups that own the pool
+  // (they wait before every next read) — either way nobody returns a chunk until the 20 s patience runs out (MAPAD_ELIMIT).
+  MAPAD_DEV bool acquire_base(uint32_t& c_nodes, uint32_t& c_heap) const {
+    uint32_t n = MAPAD_GPOOL_EMPTY, h = MAPAD_GPOOL_EMPTY;
+    if (gl == 0) {
+      for (uint32_t w = 0; w < MAPAD_PATIENCE_MAX; ++w) {
+        n = gpool_acquire(a->pool, shard());
+        if (n != MAPAD_GPOOL_EMPTY) {
+          h = gpool_acquire(a->pool, shard());
+          if (h != MAPAD_GPOOL_EMPTY) break;
+          gpool_release(a->pool, n, shard());
+          n = MAPAD_GPOOL_EMPTY;
+        }
+        dev_backoff<G>();
+      }
+    }
+    c_nodes = Grp<G>::shfl(n, 0);
+    c_heap = Grp<G>::shfl(h, 0);
+    return c_heap != MAPAD_GPOOL_EMPTY;
+  }
   MAPAD_DEV bool ensure_node(uint32_t id) {
     if (id >= a->max_nodes) return false;
     const uint32_t c = id >> NPC_SHIFT;
@@ -872,14 +895,9 @@ MAPAD_DEV void group_search_lane(const GroupLaunch<WIDE>& a, uint32_t slot, int 
   ws.slot = slot;
   ws.gl = gl;
   // every group takes its two base chunks (nodes, heap) from the device-wide pool when it starts and returns them when it exits
-  ws.frames = MAPAD_PATIENCE_MAX;  // full patience while waiting for the base chunks
-  const uint32_t c_nodes = ws.acquire_chunk();
-  const uint32_t c_heap = c_nodes != MAPAD_GPOOL_EMPTY ? ws.acquire_chunk() : MAPAD_GPOOL_EMPTY;
-  if (c_heap == MAPAD_GPOOL_EMPTY) {
-    if (gl == 0) {
-      if (c_nodes != MAPAD_GPOOL_EMPTY) gpool_release(a.pool, c_nodes, ws.shard());
-      dev_atomic_or(&a.cur->overflow, MAPAD_POOL_TIMEOUT_FLAG);
-    }
+  uint32_t c_nodes, c_heap;
+  if (!ws.acquire_base(c_nodes, c_heap)) {
+    if (gl == 0) dev_atomic_or(&a.cur->overflow, MAPAD_POOL_TIMEOUT_FLAG);
     return;
   }
   if (gl == 0) { ws.table()[0] = c_nodes; ws.table()[a.nt] = c_heap; }

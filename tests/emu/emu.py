@@ -47,12 +47,12 @@ def lib():
     return _lib
 
 
-def map_batch(index, params, seqs=None, quals=None, seeds=None, cap=1 << 16, layout=-1, packed=None, group=None):
+def map_batch(index, params, seqs=None, quals=None, seeds=None, cap=1 << 16, layout=-1, packed=None, group=None, custom_penalties=None):
     """group=None: the per-thread reference loop (search_core.cuh::search_read); group=dict(G=8, n_groups=3, pool_chunks=64, lpt=1):
-    the group kernel of search_group.cuh under the SIMT emulator."""
+    the group kernel of search_group.cuh under the SIMT emulator.  custom_penalties: MAPAD_MODEL_CUSTOM's precomputed table."""
     if packed is None:
         packed = abi.pack_reads(seqs, quals)
-    R, keep = api.make_reads(packed[0], packed[1], packed[2], seeds)
+    R, keep = api.make_reads(packed[0], packed[1], packed[2], seeds, custom_penalties)
     h = C.c_void_p()
     if group is None:
         rc = lib().emu_map_batch(index.h, C.byref(params), C.byref(R), cap, layout, C.byref(h))
