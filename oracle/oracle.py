@@ -47,6 +47,7 @@ def lib():
             "ora_index_occ": (u64, [vp, u64, u8]),
             "ora_index_sa_get": (i32, [vp, u64, C.POINTER(u64)]),
             "ora_index_extend": (None, [vp, u64, u64, u64, C.POINTER(u64)]),
+            "ora_verify_index": (i32, [vp, u64, vp, vp, vp, u64, u64, vp, u64, i32, C.c_char_p, u64]),
             "ora_params_new": (vp, []),
             "ora_params_free": (None, [vp]),
             "ora_params_model_simple": (None, [vp, i32, f32, f32, f32, f32, f32, i32]),
@@ -206,6 +207,77 @@ class OracleIndex:
     def positions(self, lower, size):
         """Interval::occ(&suffix_array): text positions of SA rows [lower, lower+size)."""
         return [self.sa_get(r) for r in range(lower, lower + size)]
+
+    def arrays(self):
+        """The index in the layout of mapad_b200.api.Index.arrays() (`less` padded to 8 entries)."""
+        n = self.n
+        less = self.less()
+        orig = self.original_symbols()
+        return dict(n=n, bwt=self.bwt(), less=less + [n] * (8 - len(less)), sentinel_rows=self.sentinel_rows(),
+                    sa_sample=self.sa_samples(), sa_rate=32,
+                    extra_rows=np.array(self.extra_rows(), dtype=np.uint64).reshape(-1, 2),
+                    orig_pos=np.array(sorted(orig), dtype=np.uint64), orig_sym=np.array([orig[k] for k in sorted(orig)], dtype=np.uint8))
+
+
+class IndexMismatch(AssertionError):
+    """verify_index found that the arrays are not the index of the text."""
+
+
+_RANK = np.zeros(256, dtype=np.uint8)  # 0: not a base
+for _c, _r in zip(b"ACGTacgt", (1, 2, 3, 4, 1, 2, 3, 4)):
+    _RANK[_c] = _r
+_COMP_RANK = np.array([0, 4, 3, 2, 1, 5], dtype=np.uint8)
+
+
+def text_ranks(seqs):
+    """The rank text `fwd $ revcomp $` ($ = 0, A C G T = 1..4, X = 5) of the contig sequences `seqs` (str, bytes or uint8
+    arrays, concatenated in order), as `mapad index` builds it: a run of >= 20 equal non-ACGT symbols becomes X.  Shorter
+    runs are replaced by seeded draws that cannot be reproduced independently, so they are refused (ValueError)."""
+    parts = [np.frombuffer(s.encode() if isinstance(s, str) else s, dtype=np.uint8) if not isinstance(s, np.ndarray) else s
+             for s in seqs]
+    g = parts[0] if len(parts) == 1 else np.concatenate(parts)
+    G = len(g)
+    out = np.empty(2 * G + 2, dtype=np.uint8)
+    fwd = out[:G]
+    np.take(_RANK, g, out=fwd)
+    other = np.flatnonzero(fwd == 0)
+    if len(other):
+        sym = np.char.upper(g[other].view("S1")).view(np.uint8)
+        # runs of one symbol over consecutive positions (runs cross contig boundaries, as in the indexer)
+        new_run = np.ones(len(other), dtype=bool)
+        new_run[1:] = (np.diff(other) != 1) | (sym[1:] != sym[:-1])
+        run_id = np.cumsum(new_run) - 1
+        run_len = np.bincount(run_id)
+        short = run_len[run_id] < 20
+        if short.any():
+            raise ValueError("a run of %d non-ACGT symbols at %d is replaced by seeded draws" % (run_len[run_id[short][0]], other[short][0]))
+        fwd[other] = 5
+    out[G] = 0
+    np.take(_COMP_RANK, fwd[::-1], out=out[G + 1:2 * G + 1])
+    out[-1] = 0
+    return out
+
+
+def verify_index(text, arrays, n_threads=None):
+    """Checks index arrays (the layout of mapad_b200.api.Index.arrays()) against the rank text from text_ranks() with the
+    oracle's independent LF-walk verifier.  Raises IndexMismatch naming a wrong row."""
+    a = arrays
+    text = np.ascontiguousarray(text, dtype=np.uint8)
+    bwt = np.ascontiguousarray(a["bwt"], dtype=np.uint8)
+    if len(text) != a["n"] or len(bwt) != a["n"]:
+        raise IndexMismatch("text of %d symbols, index of n = %d with %d BWT rows" % (len(text), a["n"], len(bwt)))
+    less = np.ascontiguousarray(a["less"], dtype=np.uint64)
+    if len(less) != 8:
+        raise IndexMismatch("less has %d entries, expected 8" % len(less))
+    ss = np.ascontiguousarray(a["sa_sample"], dtype=np.uint64)
+    if len(ss) == 0:
+        raise IndexMismatch("no SA samples")
+    extra = np.ascontiguousarray(a["extra_rows"], dtype=np.uint64).reshape(-1)
+    msg = C.create_string_buffer(512)
+    rc = lib().ora_verify_index(_ptr(text), len(text), _ptr(bwt), _ptr(less), _ptr(ss), len(ss), a["sa_rate"], _ptr(extra), len(extra) // 2,
+                                n_threads or os.cpu_count() or 1, msg, len(msg))
+    if rc:
+        raise IndexMismatch(msg.value.decode())
 
 
 class OracleParams:

@@ -4,6 +4,8 @@
 #include "oracle.hpp"
 
 #include <atomic>
+#include <cstdarg>
+#include <mutex>
 #include <thread>
 
 #include "../include/mapad_gpu.h"
@@ -97,6 +99,214 @@ void map_one(const Index& ix, const Params& p, const uint8_t* seq, const uint8_t
   out.xa = r.xa;
 }
 
+// Runs f(lo, hi) over [0, n_items) in slices of `grain` on n_threads threads.
+template <class F>
+void parallel_slices(uint64_t n_items, uint64_t grain, int n_threads, F f) {
+  std::atomic<uint64_t> next(0);
+  auto worker = [&]() {
+    for (;;) {
+      uint64_t lo = next.fetch_add(grain);
+      if (lo >= n_items) break;
+      f(lo, std::min(lo + grain, n_items));
+    }
+  };
+  std::vector<std::thread> th;
+  for (int t = 1; t < n_threads; ++t) th.emplace_back(worker);
+  worker();
+  for (auto& t : th) t.join();
+}
+
+// First failure of a parallel check; later ones are dropped.
+struct Failure {
+  std::atomic<bool> hit{false};
+  std::mutex mu;
+  std::string what;
+  void set(const char* fmt, ...) __attribute__((format(printf, 2, 3))) {
+    char buf[512];
+    va_list ap;
+    va_start(ap, fmt);
+    vsnprintf(buf, sizeof buf, fmt, ap);
+    va_end(ap);
+    std::lock_guard<std::mutex> g(mu);
+    if (!hit.load()) { what = buf; hit.store(true); }
+  }
+};
+
+// Sets bit i; returns whether it was already set.
+inline bool test_and_set(std::vector<uint64_t>& bits, uint64_t i) {
+  const uint64_t m = 1ull << (i & 63);
+  return __atomic_fetch_or(&bits[i >> 6], m, __ATOMIC_RELAXED) & m;
+}
+
+// #c in bwt[0, r) for c = 1..5: u64 totals every 2^32 rows, u32 counts relative to them every 64 rows.
+struct RankTable {
+  static constexpr int SYMS = 5;
+  const uint8_t* bwt;
+  std::vector<uint64_t> super;
+  std::vector<uint32_t> block;
+  uint64_t rank(uint8_t c, uint64_t r) const {
+    uint64_t k = super[(r >> 32) * SYMS + c - 1] + block[(r >> 6) * SYMS + c - 1];
+    for (uint64_t j = r & ~63ull; j < r; ++j) k += bwt[j] == c;
+    return k;
+  }
+};
+
+int verify_index(const uint8_t* text, uint64_t n, const uint8_t* bwt, const uint64_t* less, const uint64_t* sa_sample,
+                 uint64_t n_samples, uint64_t rate, const uint64_t* extra_kv, uint64_t n_extra, int n_threads, std::string* msg) {
+  Failure fail;
+  auto failed = [&]() { *msg = fail.what; return 1; };
+  if (n < 4 || n % 2 || n_threads < 1 || rate < 1) { *msg = "bad arguments"; return 1; }
+  const uint64_t G = (n - 2) / 2;
+  if (text[G] != 0 || text[n - 1] != 0) { *msg = "text is not fwd $ revcomp $"; return 1; }
+  // symbol counts of the text and of the BWT, and the BWT's '$' rows
+  const uint64_t n_blocks = (n + 63) / 64;
+  RankTable rt{bwt, std::vector<uint64_t>(((n >> 32) + 1) * RankTable::SYMS), std::vector<uint32_t>(n_blocks * RankTable::SYMS)};
+  std::mutex mu;
+  uint64_t text_cnt[8] = {0}, bwt_cnt[8] = {0};
+  std::vector<uint64_t> dollar_rows;
+  parallel_slices(n_blocks, 1 << 14, n_threads, [&](uint64_t lo, uint64_t hi) {
+    uint64_t tc[8] = {0}, bc[8] = {0};
+    std::vector<uint64_t> dr;
+    for (uint64_t b = lo; b < hi; ++b) {
+      uint64_t in_block[8] = {0};
+      for (uint64_t i = b * 64; i < std::min(n, b * 64 + 64); ++i) {
+        tc[text[i] & 7] += 1;
+        if (text[i] > 5) fail.set("text[%llu] = %u is not a symbol rank", (unsigned long long)i, text[i]);
+        in_block[bwt[i] & 7] += 1;
+        if (bwt[i] > 5) fail.set("row %llu: bwt = %u is not a symbol rank", (unsigned long long)i, bwt[i]);
+        if (bwt[i] == 0) dr.push_back(i);
+      }
+      for (int c = 0; c < 8; ++c) bc[c] += in_block[c];
+      for (int c = 1; c <= RankTable::SYMS; ++c) rt.block[b * RankTable::SYMS + c - 1] = (uint32_t)in_block[c];
+    }
+    std::lock_guard<std::mutex> g(mu);
+    for (int c = 0; c < 8; ++c) { text_cnt[c] += tc[c]; bwt_cnt[c] += bc[c]; }
+    dollar_rows.insert(dollar_rows.end(), dr.begin(), dr.end());
+  });
+  if (fail.hit) return failed();
+  {  // block counts -> counts before each block, restarting every 2^32 rows
+    uint64_t rel[RankTable::SYMS] = {0}, total[RankTable::SYMS] = {0};
+    for (uint64_t b = 0; b < n_blocks; ++b) {
+      if ((b & ((1ull << 26) - 1)) == 0)
+        for (int s = 0; s < RankTable::SYMS; ++s) { rt.super[(b >> 26) * RankTable::SYMS + s] = total[s]; rel[s] = 0; }
+      for (int s = 0; s < RankTable::SYMS; ++s) {
+        const uint32_t v = rt.block[b * RankTable::SYMS + s];
+        rt.block[b * RankTable::SYMS + s] = (uint32_t)rel[s];
+        rel[s] += v;
+        total[s] += v;
+      }
+    }
+  }
+  if (text_cnt[0] != 2) { *msg = "text has " + std::to_string(text_cnt[0]) + " sentinels, not 2"; return 1; }
+  for (int c = 0; c < 8; ++c)
+    if (bwt_cnt[c] != text_cnt[c]) {
+      fail.set("bwt holds %llu symbols of rank %d, the text %llu", (unsigned long long)bwt_cnt[c], c, (unsigned long long)text_cnt[c]);
+      return failed();
+    }
+  {
+    uint64_t acc = 0;
+    for (int c = 0; c < 8; ++c) {
+      if (less[c] != acc) {
+        fail.set("less[%d] = %llu, but the text has %llu symbols below rank %d", c, (unsigned long long)less[c], (unsigned long long)acc, c);
+        return failed();
+      }
+      acc += text_cnt[c];
+    }
+  }
+  // sampled rows and the unsampled '$' rows
+  if (n_samples != (n + rate - 1) / rate) { fail.set("%llu SA samples, expected %llu", (unsigned long long)n_samples, (unsigned long long)((n + rate - 1) / rate)); return failed(); }
+  if (sa_sample[0] != n - 1) { fail.set("row 0: SA sample = %llu, expected n - 1 = %llu", (unsigned long long)sa_sample[0], (unsigned long long)(n - 1)); return failed(); }
+  std::vector<uint64_t> extra_rows, extra_pos;
+  for (uint64_t i = 0; i < n_extra; ++i) {
+    const uint64_t r = extra_kv[2 * i], p = extra_kv[2 * i + 1];
+    if (r >= n || p >= n || r % rate == 0 || bwt[r] != 0 || (i && r <= extra_rows.back())) {
+      fail.set("extra row %llu (text position %llu): not an unsampled '$' row in increasing order", (unsigned long long)r, (unsigned long long)p);
+      return failed();
+    }
+    extra_rows.push_back(r);
+    extra_pos.push_back(p);
+  }
+  for (uint64_t r : dollar_rows)
+    if (r % rate != 0 && !std::binary_search(extra_rows.begin(), extra_rows.end(), r)) {
+      fail.set("row %llu: unsampled '$' row missing from the extra rows", (unsigned long long)r);
+      return failed();
+    }
+  // start rows: the samples, the extra rows and row 1 (the first sentinel's suffix G, which no LF step reaches)
+  const bool start_row1 = rate > 1;
+  const uint64_t n_starts = n_samples + n_extra + (start_row1 ? 1 : 0);
+  auto start = [&](uint64_t k, uint64_t* r, uint64_t* p) {
+    if (k < n_samples) { *r = k * rate; *p = sa_sample[k]; }
+    else if (k < n_samples + n_extra) { *r = extra_rows[k - n_samples]; *p = extra_pos[k - n_samples]; }
+    else { *r = 1; *p = G; }
+  };
+  auto known = [&](uint64_t r, uint64_t* p) {
+    if (r % rate == 0) { *p = sa_sample[r / rate]; return true; }
+    if (r == 1) { *p = G; return true; }
+    auto it = std::lower_bound(extra_rows.begin(), extra_rows.end(), r);
+    if (it != extra_rows.end() && *it == r) { *p = extra_pos[it - extra_rows.begin()]; return true; }
+    return false;
+  };
+  std::vector<uint64_t> row_seen(n_blocks, 0), pos_seen(n_blocks, 0);
+  enum { GOING, DONE, FAILED };
+  // one LF step of a walk at row r, text position p
+  auto step = [&](uint64_t& r, uint64_t& p) -> int {
+    if (p >= n) { fail.set("row %llu: SA = %llu is past the text end", (unsigned long long)r, (unsigned long long)p); return FAILED; }
+    if (test_and_set(row_seen, r)) { fail.set("row %llu reached twice (text position %llu)", (unsigned long long)r, (unsigned long long)p); return FAILED; }
+    if (test_and_set(pos_seen, p)) { fail.set("text position %llu reached twice (row %llu)", (unsigned long long)p, (unsigned long long)r); return FAILED; }
+    const uint8_t c = bwt[r], want = text[p ? p - 1 : n - 1];
+    if (c != want) {
+      fail.set("row %llu (text position %llu): bwt = %u, but the text before it is %u", (unsigned long long)r, (unsigned long long)p, c, want);
+      return FAILED;
+    }
+    if (c == 0) return DONE;
+    const uint64_t from = r;
+    r = less[c] + rt.rank(c, r);
+    p -= 1;
+    uint64_t kp;
+    if (r >= n) { fail.set("row %llu: LF leaves the table (%llu)", (unsigned long long)from, (unsigned long long)r); return FAILED; }
+    if (known(r, &kp)) {
+      if (kp != p) {
+        fail.set("row %llu: SA = %llu, but LF from row %llu reaches it at text position %llu", (unsigned long long)r, (unsigned long long)kp,
+                 (unsigned long long)from, (unsigned long long)p);
+        return FAILED;
+      }
+      return DONE;
+    }
+    __builtin_prefetch(&bwt[r]);
+    __builtin_prefetch(&rt.block[(r >> 6) * RankTable::SYMS]);
+    __builtin_prefetch(&row_seen[r >> 6]);
+    return GOING;
+  };
+  // each thread advances W walks in turn, so that the cache misses of one step overlap with the others' work
+  parallel_slices(n_starts, 4096, n_threads, [&](uint64_t lo, uint64_t hi) {
+    constexpr int W = 16;
+    uint64_t wr[W], wp[W];
+    int live = 0;
+    for (; live < W && lo < hi; ++live) start(lo++, &wr[live], &wp[live]);
+    while (live > 0) {
+      if (fail.hit.load(std::memory_order_relaxed)) return;
+      for (int i = 0; i < live;) {
+        const int s = step(wr[i], wp[i]);
+        if (s == FAILED) return;
+        if (s == DONE) {
+          if (lo < hi) start(lo++, &wr[i], &wp[i]);
+          else { wr[i] = wr[live - 1]; wp[i] = wp[live - 1]; --live; continue; }
+        }
+        ++i;
+      }
+    }
+  });
+  if (fail.hit) return failed();
+  for (uint64_t b = 0; b < n_blocks; ++b) {
+    const uint64_t full = b + 1 < n_blocks || n % 64 == 0 ? ~0ull : (1ull << (n % 64)) - 1;
+    if (row_seen[b] != full) {
+      fail.set("row %llu is not reached from any sampled row", (unsigned long long)(b * 64 + __builtin_ctzll(~row_seen[b])));
+      return failed();
+    }
+  }
+  return 0;
+}
+
 }  // namespace
 
 extern "C" {
@@ -150,6 +360,20 @@ uint64_t ora_index_original_symbols(void* h, uint64_t* pos_out, uint8_t* sym_out
   return i;
 }
 uint64_t ora_index_occ(void* h, uint64_t r, uint8_t a) { return ((Index*)h)->occ(r, a); }
+// Independent check of a BWT + sampled SA (any builder's) against the rank text `fwd $ revcomp $` ($ = 0, A..T = 1..4,
+// X = 5).  It walks LF from every row whose text position is known (the sampled rows, the extra rows and row 1, the first
+// sentinel's suffix) to the next known row or '$' row: each row it passes must hold the text symbol before its position,
+// each row and each position must be reached exactly once, and every known row must be reached at its own position.
+// With `less` equal to the text's symbol counts, these local conditions force the suffix order.  Uses its own rank
+// table, no Index.  Returns 0 if the arrays are the index of `text`, else 1 and a message naming a wrong row.
+int ora_verify_index(const uint8_t* text, uint64_t n, const uint8_t* bwt, const uint64_t* less8, const uint64_t* sa_sample,
+                     uint64_t n_samples, uint64_t sa_rate, const uint64_t* extra_kv, uint64_t n_extra, int n_threads, char* msg,
+                     uint64_t cap) {
+  std::string m;
+  int rc = verify_index(text, n, bwt, less8, sa_sample, n_samples, sa_rate, extra_kv, n_extra, n_threads, &m);
+  snprintf(msg, cap, "%s", m.c_str());
+  return rc;
+}
 int ora_index_sa_get(void* h, uint64_t row, uint64_t* out) { usize v = 0; bool ok = ((Index*)h)->sa_get(row, &v, nullptr); *out = v; return ok; }
 void ora_index_extend(void* h, uint64_t lower, uint64_t lower_rev, uint64_t size, uint64_t* out12) {
   BiInterval o[4];

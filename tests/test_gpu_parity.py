@@ -248,17 +248,27 @@ def test_cfg5_cell(api):
     m.close()
 
 
-def test_real_wide_index(api):
+def test_real_wide_index(api, capfd):
     """A reference whose text (2 G + 2 symbols) exceeds 2^32 rows: device suffix sorter, 64-byte occ blocks, u64 SA samples,
     40-bit tree nodes.  Reads from both strands, reads that straddle a contig boundary (must not be reported there), and
-    rows / positions beyond 2^32."""
+    rows / positions beyond 2^32.  The oracle maps on the device's own arrays, so they are first checked against the text
+    by the independent verifier."""
+    import time
     from mapad_b200 import workloads
+    from sorter_cases import FALLBACK_MESSAGE
     gbp = 2_200_000_000
     genome = workloads.random_genome_array(gbp, seed=42)
     contigs = workloads.split_contigs(genome, 24)
+    capfd.readouterr()
     index = api.Index.build(contigs, device=0)
+    assert FALLBACK_MESSAGE not in capfd.readouterr().err
+    del contigs
     a = index.arrays()
     assert a["n"] == 2 * gbp + 2 and a["n"] > 1 << 32
+    t0 = time.time()
+    ora.verify_index(ora.text_ranks([genome]), a)
+    with capfd.disabled():
+        print("\nverify_index: %d rows in %.1f s on %d threads" % (a["n"], time.time() - t0, os.cpu_count() or 1))
     oix = ora.OracleIndex.from_arrays(a["bwt"], a["sa_sample"], a["sa_rate"], a["extra_rows"], a["contigs"], a["orig_pos"], a["orig_sym"])
     del a
     spec = cli_params("single_stranded")
@@ -290,21 +300,26 @@ def test_real_wide_index(api):
             assert abs(int(rec["absolute_pos"][k]) - (cuts[k % 23 + 1] - L // 2)) > L, k
 
 
-def test_device_index_builder_matches_host(api):
+def test_device_index_builder_matches_host(api, capfd):
     """mapad_index_build_on_device (prefix-key radix sort on the GPU) must produce exactly the arrays of the host
     SA-IS builder; a repetitive text makes it fall back to the host builder (still identical)."""
+    from sorter_cases import FALLBACK_MESSAGE
     for gsize, seed in ((300_000, 7), (65_537, 8)):
         genome = random_genome(gsize, seed=seed)
         contigs = [("a", genome[: gsize // 2]), ("b", genome[gsize // 2:])]
         host = api.Index.build(contigs).arrays()
+        capfd.readouterr()
         dev = api.Index.build(contigs, device=0).arrays()
+        assert FALLBACK_MESSAGE not in capfd.readouterr().err  # sorted on the device
         assert host["n"] == dev["n"] and host["less"] == dev["less"] and host["sentinel_rows"] == dev["sentinel_rows"]
         assert np.array_equal(host["bwt"], dev["bwt"])
         assert np.array_equal(host["sa_sample"], dev["sa_sample"])
         assert np.array_equal(host["extra_rows"], dev["extra_rows"])
     rep = [("r", "ACGT" * 200 + "N" * 30 + "GATTACA" * 50)]
     host = api.Index.build(rep).arrays()
+    capfd.readouterr()
     dev = api.Index.build(rep, device=0).arrays()
+    assert FALLBACK_MESSAGE in capfd.readouterr().err
     assert np.array_equal(host["bwt"], dev["bwt"]) and np.array_equal(host["sa_sample"], dev["sa_sample"])
 
 
